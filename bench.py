@@ -2,6 +2,7 @@
 """bench.py — story-turns/sec of the SEED-Story interleaved inference hot path on B200 (contract in the task brief).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config story|sink|sdxl] [--stories-per-gpu S]
+                  [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 ... bench.py --gpus N ...
 
 --config story (default; BASELINE.json configs[1], and configs[2] when launched on N GPUs): a *step* is one 10-turn
@@ -113,6 +114,44 @@ def ev():
     return torch.cuda.Event(enable_timing=True)
 
 
+DUMP_BYTES = 60 * 10 ** 6     # payload bound of --dump-outputs (the .npy headers stay far inside 64 MB)
+
+
+def dump_outputs(outdir, last):
+    """--dump-outputs: what the last timed step returned to its caller, as float32 .npy files in `outdir`.
+      generate_ids.npy [n, L]    every turn's generated ids (stories in order, then turns), padded with -1
+      has_img_output.npy [n]     1 where the turn produced an image
+      images.npy [m, K]          the m uint8 1024x1024x3 images, flattened; all of each image when they fit the bound,
+                                 else the same K positions of each (torch.randperm, seed 0), listed in image_index.npy
+    The bench inputs and weights are seeded, so two builds run with the same arguments can be compared file by file."""
+    import numpy as np
+    turns = last.get("turns", [])
+    images = last.get("images", [o["image"] for o in turns if o["image"] is not None])
+    arrays = {}
+    if turns:
+        width = max(len(o["generate_ids"]) for o in turns)
+        ids = np.full((len(turns), width), -1, np.float32)
+        for r, o in enumerate(turns):
+            ids[r, :len(o["generate_ids"])] = o["generate_ids"]
+        arrays["generate_ids"] = ids
+        arrays["has_img_output"] = np.array([o["has_img_output"] for o in turns], np.float32)
+    if images:
+        numel = images[0].numel()
+        room = (DUMP_BYTES - sum(a.nbytes for a in arrays.values())) // 4
+        flat = [im.reshape(-1) for im in images]
+        if numel * len(images) <= room:
+            arrays["images"] = torch.stack(flat).float().cpu().numpy()
+        else:
+            k = room // (len(images) + 1)
+            idx = torch.randperm(numel, generator=torch.Generator().manual_seed(0))[:k].sort().values
+            idx_dev = idx.to(images[0].device)
+            arrays["images"] = torch.stack([f[idx_dev] for f in flat]).float().cpu().numpy()
+            arrays["image_index"] = idx.float().numpy()      # exact: numel < 2^24
+    os.makedirs(outdir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(outdir, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------
 # our arm
 # ------------------------------------------------------------------------------------------------
@@ -153,6 +192,10 @@ def run_ours(args):
     n_steps_total = args.warmup + args.steps
     host_img = torch.empty((1024, 1024, 3), dtype=torch.uint8).pin_memory()
     counters = dict(h2d=0, d2h=0)
+    last = {}      # what the last timed step returned, kept for --dump-outputs
+
+    def keep(i):
+        return args.dump_outputs is not None and i == n_steps_total - 1
 
     if args.config in ("story", "sink"):
         turns, sink, spg = args.turns, args.config == "sink", max(1, args.stories_per_gpu)
@@ -168,7 +211,9 @@ def run_ours(args):
 
         def step_dev(i):
             grp = dev_inputs[i * spg:(i + 1) * spg]
-            outs = run([g[0] for g in grp], [g[1] for g in grp])
+            outs = run([g[0] for g in grp], [g[1] for g in grp], return_images=keep(i))
+            if keep(i):
+                last["turns"] = [o for st in outs for o in st]
             return sum(1 for st in outs for o in st if o["has_img_output"])   # a story ends early if a turn emits no image
 
         def step_e2e(i):
@@ -200,7 +245,9 @@ def run_ours(args):
                                          output_type="pt", input_image_size=448)[0]
 
         def step_dev(i):
-            sdxl_image(dev_feats[i])
+            img = sdxl_image(dev_feats[i])
+            if keep(i):
+                last["images"] = [img]
             return 1
 
         def step_e2e(i):
@@ -231,6 +278,9 @@ def run_ours(args):
     ms = max_over_ranks(e0.elapsed_time(e1))
     clocks = sampler.stop() if rank == 0 else None
     value = sum_over_ranks(n_units) / (ms * 1e-3)
+    if args.dump_outputs is not None and rank == 0:
+        dump_outputs(args.dump_outputs, last)
+    last.clear()
 
     # ---- e2e: host buffers, H2D + D2H inside the timed region --------------------------------------
     # (same steps, same inputs; bounded to args.e2e_steps of them so the whole default run stays within minutes)
@@ -673,12 +723,16 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=6, help="steps of the host-buffer (e2e) leg, <= --steps")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-eager-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="after the timed steps, write what the last "
+                    "timed step returned (rank 0) as DIR/<name>.npy, float32, under 64 MB in all (see dump_outputs)")
     args = ap.parse_args()
     if args.turns is None:
         args.turns = 25 if args.config == "sink" else TURNS
     if args.denoise_steps is None:
         args.denoise_steps = 30 if args.config == "sdxl" else DENOISE_STEPS
     if args.impl == "reference":
+        if args.dump_outputs is not None:
+            ap.error("--dump-outputs: the reference arm times oracle pieces and returns no story outputs")
         run_reference(args)
     else:
         run_ours(args)

@@ -1,8 +1,8 @@
 """Acceptance: the reference's own inference scripts run UNCHANGED on top of the drop-in `src.*` package.
 
 `src/inference/gen_george.py` and `src/inference/vis_george_sink.py` are executed with runpy exactly as shipped
-(`__graft_entry__.build()` stages unmodified copies from /root/reference into the git-ignored baseline/_ref/, the
-same place the contract's reference install goes; /root/reference does not exist on the GPU box).  Everything they
+(`__graft_entry__.build()` stages unmodified copies from a reference checkout into the git-ignored oracle/_ref/,
+oracle/stage_reference.py; the scripts are never committed, so the tests skip where none were staged).  Everything they
 touch is resolved as in a real checkout: hydra `_target_` paths -> the drop-in modules, `transformers.LlamaTokenizer`
 from a tokenizer directory, HF / diffusers / torch checkpoints from `pretrained/…`, `data/json/val.jsonl`, and they
 write `output/val_0/NN.jpg`.  Widths are reduced (tests/acceptance_fixture.py); resolutions, token counts, the
@@ -15,11 +15,12 @@ import sys
 
 import pytest
 
+from oracle.stage_reference import STAGED as SCRIPTS
+
 pytestmark = pytest.mark.gpu
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 PKG = os.path.join(ROOT, "seed-story_b200")
-SCRIPTS = os.path.join(ROOT, "baseline", "_ref", "src", "inference")
 
 
 @pytest.fixture(scope="module")
@@ -42,7 +43,7 @@ def _run_script(name, project):
     root, stubs, _ = project
     script = os.path.join(SCRIPTS, name)
     if not os.path.exists(script):
-        pytest.skip(f"{script} not staged (run __graft_entry__.build() where /root/reference exists)")
+        pytest.skip(f"{script} not staged (__graft_entry__.build() stages it where a reference checkout is readable)")
     env = dict(os.environ)
     env["PYTHONPATH"] = os.pathsep.join([os.path.join(PKG, "shims"), PKG, stubs, env.get("PYTHONPATH", "")])
     env["SEEDSTORY_PROJECT_ROOT"] = PKG          # pyrootutils.setup_root(): the reference tree has no .project-root
